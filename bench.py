@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — scenes/sec (256×256×32 voxels @10 % occupancy) forward+backward, the BASELINE.json metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|bf16] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -17,6 +17,8 @@ Two timed regions, both bracketed by barrier + cuda.synchronize and CUDA events:
           (asynchronous D2H into pinned memory) every step.
 `--impl reference` times the CPU restatement of the MinkowskiEngine algorithm (oracle/) on the host
 cores on a bounded crop of the same workload (ME 0.5.4 itself is not installable offline, BASELINE.md §2).
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (see dump_outputs); scenes and initial
+weights are seeded, so runs with the same arguments get the same inputs and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,6 +37,7 @@ sys.path.insert(0, ROOT)
 os.environ.setdefault("PYTORCH_CUDA_ALLOC_CONF", "expandable_segments:True")   # scene sizes vary step to step
 import faulthandler  # noqa: E402
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -171,6 +174,67 @@ def h2d_bytes(scene):
     return n
 
 
+DUMP_BUDGET = 64 << 20          # bytes written by --dump-outputs, all files together
+DUMP_PARAM_SAMPLE = 1 << 20     # entries of the flattened parameters (and of their gradients) written
+
+
+def _named_outputs(prefix, v, acc):
+    """Flattens the network's output structure into {"sem_logits_at_scales.4.0": tensor-or-SparseTensor, ...}."""
+    if isinstance(v, dict):
+        for k, x in v.items():
+            _named_outputs(f"{prefix}{k}.", x, acc)
+    elif isinstance(v, (list, tuple)):
+        for i, x in enumerate(v):
+            _named_outputs(f"{prefix}{i}.", x, acc)
+    elif isinstance(v, torch.Tensor) or (hasattr(v, "F") and hasattr(v, "C")):
+        acc[prefix[:-1]] = v
+
+
+def dump_outputs(path, out, loss, params):
+    """Writes one step's results as path/<name>.npy: `loss` (float64), every dense output tensor (float32), and for every
+    sparse output `<name>.coords` (float64 [R, 4], batch x y z) and `<name>.feats` (float32 [R, C]).  Sparse rows are sorted
+    by coordinate; a large output keeps the rows whose coordinates hash lowest, so two builds keep the same voxels where
+    their coordinate sets agree.  `params_sample` / `grads_sample` (float32) are the parameters after the optimiser step
+    and their gradients at 2^20 positions of the flattened parameter list drawn with a fixed seed.
+
+    The dumped step follows W + SETTLE + 2K optimiser steps, and AdamW and the argmax pruning amplify any difference in
+    the last bit.  The engine's float reductions sum their partials in a fixed order; the BatchNorm statistics still
+    accumulate in float64 atomics, whose order can change the float64 sum's last bit but only rarely the float result.
+    Two runs with the same arguments on the same GPU therefore normally write the same arrays."""
+    named = {}
+    _named_outputs("", out, named)
+    sparse = {k: v for k, v in named.items() if not isinstance(v, torch.Tensor)}
+    dense = {k: v for k, v in named.items() if isinstance(v, torch.Tensor)}
+    # rows per sparse output such that they fit the budget left by the loss, the dense outputs and the two samples
+    fixed = 8 + sum(4 * v.numel() for v in dense.values()) + 2 * 4 * DUMP_PARAM_SAMPLE
+    row_bytes = sum(8 * 4 + 4 * v.F.shape[1] for v in sparse.values())
+    max_rows = max(1, (DUMP_BUDGET - fixed) // max(row_bytes, 1))
+    arrays = {"loss": loss.detach().double().cpu().numpy().reshape(1)}
+    for k, v in dense.items():
+        arrays[k] = v.detach().float().cpu().numpy()
+    for k, v in sparse.items():
+        c = v.C.detach().long().cpu()
+        key = (((c[:, 0] + 32768) << 48) | ((c[:, 1] + 32768) << 32) | ((c[:, 2] + 32768) << 16) | (c[:, 3] + 32768)).numpy()
+        rows = np.arange(len(key))
+        if len(key) > max_rows:
+            h = key.astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15)       # wraps mod 2^64: a fixed scramble of the key
+            rows = np.argpartition(h, max_rows - 1)[:max_rows]
+        rows = rows[np.argsort(key[rows], kind="stable")]
+        arrays[f"{k}.coords"] = c.numpy()[rows].astype(np.float64)
+        arrays[f"{k}.feats"] = v.F.detach().float().cpu().numpy()[rows]
+    flat_p = torch.cat([p.detach().reshape(-1).float() for p in params])
+    flat_g = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1).float() for p in params])
+    idx = torch.randint(0, flat_p.numel(), (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort()[0]
+    arrays["params_sample"] = flat_p[idx.to(flat_p.device)].cpu().numpy()
+    arrays["grads_sample"] = flat_g[idx.to(flat_g.device)].cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BUDGET, f"--dump-outputs: {total} bytes > {DUMP_BUDGET}"
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
+    return total, len(arrays)
+
+
 # ------------------------------------------------------------------------------------------------------------
 def run_ours(a):
     from pasco_b200 import build
@@ -212,8 +276,9 @@ def run_ours(a):
     torch.cuda.synchronize()
     # the reference's DDP gradient averaging (scripts/train.py:213): 64 MB buckets all-reduced while backward continues
     reducer = parallel.GradReducer(params, bucket_mb=a.bucket_mb) if world > 1 else None
+    kept = {}                   # outputs of the last timed step, for --dump-outputs
 
-    def step(scene, micro=0):
+    def step(scene, micro=0, keep=False):
         """One micro-step (one MIMO group of M scenes); the optimiser step closes on the last of ACC micro-steps
         (gradient accumulation, scripts/train.py:62,203: `--accum_batch`)."""
         out = net(scene["in_feats"], scene["in_coords"], scene["global_min_Cs"], scene["global_max_Cs"],
@@ -221,6 +286,8 @@ def run_ours(a):
         loss = total_loss(out, scene, N_CLASSES, net.class_frequencies)
         if ACC > 1:
             loss = loss / ACC
+        if keep:
+            kept.update(out=out, loss=loss)
         last = micro == ACC - 1
         if micro == 0:
             if reducer is not None:
@@ -240,15 +307,15 @@ def run_ours(a):
     copy_stream = torch.cuda.Stream(device=dev)
     loss_host = torch.zeros(max(a.steps, 1), dtype=torch.float32).pin_memory()
 
-    def timed(n_steps, from_host):
+    def timed(n_steps, from_host, keep_last=False):
         gc.collect()
         gc.disable()            # no collector pauses inside the timed region (collected between regions)
         try:
-            return _timed(n_steps, from_host)
+            return _timed(n_steps, from_host, keep_last)
         finally:
             gc.enable()
 
-    def _timed(n_steps, from_host):
+    def _timed(n_steps, from_host, keep_last):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
@@ -276,7 +343,7 @@ def run_ours(a):
                 main.wait_event(ev)
                 if i + 1 < n_steps * ACC:
                     nxt = prefetch(i + 1)
-                ls = step(sc, i % ACC).detach()
+                ls = step(sc, i % ACC, keep=keep_last and i == n_steps * ACC - 1).detach()
                 if i % ACC == ACC - 1:
                     loss_host[(i // ACC) % loss_host.shape[0]].copy_(ls, non_blocking=True)   # D2H read of the result
         else:
@@ -328,8 +395,13 @@ def run_ours(a):
                 t.record_stream(main_stream)
     torch.cuda.synchronize()
     del warm
-    ms_e2e, _ = timed(a.steps, from_host=True)
+    ms_e2e, _ = timed(a.steps, from_host=True, keep_last=a.dump_outputs is not None)
     log(f"e2e region: {ms_e2e / a.steps:.1f} ms/step")
+    if a.dump_outputs is not None and rank == 0:
+        # before the profiled step below, which would replace the gradients and update the parameters again
+        n_bytes, n_files = dump_outputs(a.dump_outputs, kept["out"], kept["loss"], params)
+        log(f"wrote {n_files} arrays ({n_bytes / 2**20:.1f} MiB) of the last timed step to {a.dump_outputs}")
+    kept.clear()
     clocks = sampler.stop() if sampler else None
     # per-launch CUDA events of the conv kernels (the roofline block) come from ONE extra step of the same workload run
     # right after the timed regions (same clocks, same allocator state): recording ~260 event pairs and the pair counts
@@ -423,8 +495,8 @@ def cpu_baseline(_budget_s: float = 20.0):
 
 def run_reference(a):
     """The reference arm: the CPU restatement of the reference's MinkowskiEngine path on the host cores.  One STEP = one
-    forward+backward(+losses) pass over the fixed 1/16-scene crop (a bounded sample of config.workload); W warm-up and K
-    timed steps as asked (K is cut only if the run would exceed ~4 minutes; `steps` then reports what ran).
+    forward+backward(+losses) pass over the fixed 1/16-scene crop (a bounded sample of config.workload); W warm-up
+    (at least 1, at most 2) and exactly K timed steps.
     value = (1/16 scene) / median step time — the linear-in-voxels scaling is stated in config.workload;
     `--ref-full-scene` adds ONE unscaled full-scene pass (minutes) as `full_scene`."""
     rank = int(os.environ.get("RANK", "0"))
@@ -434,15 +506,11 @@ def run_reference(a):
     import net_oracle
     cores = min(os.cpu_count(), 32)
     torch.set_num_threads(cores)
-    t0 = time.time()
     n_warm = max(1, min(a.warmup, 2))
-    probe = net_oracle.time_crop(repeats=1, warmup=n_warm)
-    per = probe["seconds"]
-    k_run = int(max(3, min(max(1, a.steps), (240.0 - (time.time() - t0)) / max(per, 1e-3))))
-    r = net_oracle.time_crop(repeats=k_run, warmup=0)
+    r = net_oracle.time_crop(repeats=a.steps, warmup=n_warm)
     v = r["scenes_per_s"]
     line = {"impl": "reference", "metric": METRIC, "value": round(v, 6), "unit": "scenes/s", "n_gpus": a.gpus,
-            "steps": k_run, "steps_requested": a.steps, "warmup": n_warm,
+            "steps": a.steps, "warmup": n_warm,
             "ms_per_step": round(r["seconds"] * 1e3, 1), "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": "configs[1] shape: 256x256x32 @10% occ, full PaSCo fwd+bwd+losses (M=1, f=64); each STEP is a "
@@ -450,7 +518,7 @@ def run_reference(a):
                                    "step time), assuming cost linear in voxels",
                        "parallelism": f"cpu x{cores} threads", "scene_fraction_per_step": 1.0 / r["div"]},
             "cpu_baseline": {"value": round(v, 6), "unit": "scenes/s", "cores": cores, "kind": "port",
-                             "sample": r["sample"].replace("0 warm-up +", f"{n_warm} warm-up + 1 probe pass (untimed) +"),
+                             "sample": r["sample"],
                              "times": r["times"], "spread": r["spread"]},
             "e2e": {"value": round(v, 6), "unit": "scenes/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     if a.ref_full_scene:
@@ -477,7 +545,11 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--bucket-mb", type=float, default=64.0, help="gradient all-reduce bucket size (N > 1)")
     ap.add_argument("--ref-full-scene", action="store_true", help="--impl reference: also time one unscaled full scene")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -172,20 +172,25 @@ int pasco_conv_forward_planes(const void* hi, const void* lo, int64_t n_in, cons
                               pasco_stream_t s);
 int pasco_conv_wgrad_planes(const void* in_hi, const void* in_lo, int64_t n_in, const int32_t* nbr, int32_t K,
                             int64_t n_out, int32_t Cin, int32_t Cout, const void* g_hi, const void* g_lo, float* dW,
-                            int32_t precision, int64_t in_pitch, int64_t gout_pitch, pasco_stream_t s);
+                            int32_t precision, int64_t in_pitch, int64_t gout_pitch, float* workspace,
+                            int64_t workspace_bytes, pasco_stream_t s);
 
-/* dW[k] = sum_o in[nbr[k,o],:]^T @ gout[o,:]   (tcgen05, MN-major operands); dW float32 [K,Cin,Cout] zeroed by caller */
+/* dW[k] = sum_o in[nbr[k,o],:]^T @ gout[o,:]   (tcgen05, MN-major operands); dW float32 [K,Cin,Cout] zeroed by caller.
+ * Both weight-gradient kernels store each CTA's partial dW in `workspace` (pasco_conv_wgrad_workspace_bytes) and add the
+ * partials in a fixed order, so dW is the same from run to run.                                                       */
+int64_t pasco_conv_wgrad_workspace_bytes(int32_t K, int64_t n_out, int32_t Cin, int32_t Cout);
 int pasco_conv_wgrad_tc(const float* in, int64_t n_in, const int32_t* nbr, int32_t K, int64_t n_out, int32_t Cin,
                         int32_t Cout, const float* gout, const float* in_scale, const float* in_shift,
                         int32_t in_act, float* dW, int32_t precision, int64_t in_pitch, int64_t gout_pitch,
-                        pasco_stream_t s);
+                        float* workspace, int64_t workspace_bytes, pasco_stream_t s);
 
 /* CUDA-core fp32 reference path of the same contraction (any Cin/Cout; validation + odd shapes) */
 int pasco_conv_forward_simt(const float* in, const int32_t* nbr, int32_t K, int64_t n_out, int32_t Cin,
                             int32_t Cout, const float* W, int32_t w_transposed, const int32_t* koff_map,
                             const float* bias, float* out, pasco_stream_t s);
+int64_t pasco_conv_wgrad_simt_workspace_bytes(int32_t K, int64_t n_out, int32_t Cin, int32_t Cout);
 int pasco_conv_wgrad_simt(const float* in, const int32_t* nbr, int32_t K, int64_t n_out, int32_t Cin, int32_t Cout,
-                          const float* gout, float* dW, pasco_stream_t s);
+                          const float* gout, float* dW, float* workspace, int64_t workspace_bytes, pasco_stream_t s);
 
 /* ---- pooling / reductions --------------------------------------------------------------------
  * ME.MinkowskiMaxPooling(k=s, stride=s) (transformer_predictor_v2.py:100-102): out rows
@@ -228,11 +233,12 @@ int64_t pasco_xattn_workspace_bytes(int32_t Q, int64_t P, int32_t H, int32_t D);
 int pasco_xattn_forward(const float* q, const float* k, const float* v, const uint32_t* mask, int32_t Q, int64_t P,
                         int32_t H, int32_t D, float scale, float* out, float* lse, float* workspace,
                         int64_t workspace_bytes, pasco_stream_t s);
-/* backward of the above: recomputes the probabilities from lse; dq [Q, H*D] ZEROED by the caller (fp32 red.add),
- * dk / dv [P, H*D] are fully overwritten (every row written exactly once, no atomics).                            */
+/* backward of the above: recomputes the probabilities from lse; dq [Q, H*D] ZEROED by the caller (the key chunks'
+ * partial dq go to `workspace`, sized by pasco_xattn_workspace_bytes, and are added in chunk order), dk / dv [P, H*D]
+ * are fully overwritten (every row written exactly once, no atomics).                                            */
 int pasco_xattn_backward(const float* q, const float* k, const float* v, const uint32_t* mask, const float* lse,
                          const float* out, const float* dout, int32_t Q, int64_t P, int32_t H, int32_t D, float scale,
-                         float* dq, float* dk, float* dv, pasco_stream_t s);
+                         float* dq, float* dk, float* dv, float* workspace, int64_t workspace_bytes, pasco_stream_t s);
 
 #ifdef __cplusplus
 }

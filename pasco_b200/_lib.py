@@ -45,10 +45,12 @@ PROTOTYPES = {
     "pasco_conv_forward_splitk": (C.c_int, [_p, _i64, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _p, _p, _i32, _p, _i32, _i64, _i64, _p, _i64, _p]),
     "pasco_split_planes": (C.c_int, [_p, _i64, _i32, _i64, _p, _p, _i32, _p, _p, _p]),
     "pasco_conv_forward_planes": (C.c_int, [_p, _p, _i64, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _p, _p, _i32, _i64, _i64, _p]),
-    "pasco_conv_wgrad_planes": (C.c_int, [_p, _p, _i64, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _i32, _i64, _i64, _p]),
-    "pasco_conv_wgrad_tc": (C.c_int, [_p, _i64, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _i32, _p, _i32, _i64, _i64, _p]),
+    "pasco_conv_wgrad_planes": (C.c_int, [_p, _p, _i64, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _i32, _i64, _i64, _p, _i64, _p]),
+    "pasco_conv_wgrad_workspace_bytes": (_i64, [_i32, _i64, _i32, _i32]),
+    "pasco_conv_wgrad_tc": (C.c_int, [_p, _i64, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _i32, _p, _i32, _i64, _i64, _p, _i64, _p]),
     "pasco_conv_forward_simt": (C.c_int, [_p, _p, _i32, _i64, _i32, _i32, _p, _i32, _p, _p, _p, _p]),
-    "pasco_conv_wgrad_simt": (C.c_int, [_p, _p, _i32, _i64, _i32, _i32, _p, _p, _p]),
+    "pasco_conv_wgrad_simt_workspace_bytes": (_i64, [_i32, _i64, _i32, _i32]),
+    "pasco_conv_wgrad_simt": (C.c_int, [_p, _p, _i32, _i64, _i32, _i32, _p, _p, _p, _i64, _p]),
     "pasco_maxpool_forward": (C.c_int, [_p, _p, _i64, _i32, _p, _p]),
     "pasco_scatter_max": (C.c_int, [_p, _p, _i64, _i32, _p, _i64, _p, _p]),
     "pasco_bn_stats": (C.c_int, [_p, _i64, _i32, _p, _p]),
@@ -58,7 +60,7 @@ PROTOTYPES = {
     "pasco_bn_bwd_reduce": (C.c_int, [_p, _p, _i64, _i32, _p, _p, _i32, _p, _p]),
     "pasco_xattn_workspace_bytes": (_i64, [_i32, _i64, _i32, _i32]),
     "pasco_xattn_forward": (C.c_int, [_p, _p, _p, _p, _i32, _i64, _i32, _i32, C.c_float, _p, _p, _p, _i64, _p]),
-    "pasco_xattn_backward": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _i64, _i32, _i32, C.c_float, _p, _p, _p, _p]),
+    "pasco_xattn_backward": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _i64, _i32, _i32, C.c_float, _p, _p, _p, _p, _i64, _p]),
     "pasco_bn_bwd_apply": (C.c_int, [_p, _p, _i64, _i32, _p, _p, _i32, _p, _p, _p, _p, _p]),
 }
 

@@ -70,6 +70,17 @@ inline int num_sms() {
   return n;
 }
 
+// out[i] += Σ_{c < n_part} part[c * stride + i], summed in slot order: a reduction whose result does not depend on which
+// CTA finished first (float atomics would make every run round differently).
+static __global__ void k_add_partials(const float* __restrict__ part, int n_part, int64_t stride, int64_t n,
+                                      float* __restrict__ out) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    float s = 0.f;
+    for (int c = 0; c < n_part; ++c) s += __ldg(part + (int64_t)c * stride + i);
+    out[i] += s;
+  }
+}
+
 inline int grid_for(int64_t work, int block, int waves = 8) {
   int64_t g = (work + block - 1) / block;
   int64_t cap = (int64_t)num_sms() * waves;

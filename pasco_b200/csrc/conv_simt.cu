@@ -90,20 +90,21 @@ extern "C" int pasco_conv_forward_simt(const float* in, const int32_t* nbr, int3
   return 0;
 }
 
-// dW[k][ci][co] = Σ_o in[nbr[k,o]][ci] * gout[o][co];  grid = (row chunks, K); fp32 atomics into dW
-constexpr int WG_ROWS = 2048;  // rows per block
+// dW[k][ci][co] = Σ_o in[nbr[k,o]][ci] * gout[o][co];  grid = (row chunks, K); each row chunk stores its partial dW in
+// part[chunk][k][ci][co], and the host sums the chunks in order (identical from run to run, unlike float atomics)
+constexpr int WG_ROWS = 2048;  // rows per block (at least)
 constexpr int WG_TILE = 16;    // rows staged per iteration
 
 __global__ void __launch_bounds__(256)
 k_wgrad_simt(const float* __restrict__ in, const int32_t* __restrict__ nbr, int64_t n_out, int Cin, int Cout,
-             const float* __restrict__ gout, float* __restrict__ dW) {
+             const float* __restrict__ gout, int64_t rows_per_block, float* __restrict__ part) {
   extern __shared__ float sm[];  // sA[WG_TILE][Cin], sG[WG_TILE][Cout]
   float* sA = sm;
   float* sG = sm + WG_TILE * Cin;
   __shared__ int sIdx[WG_TILE];
   int k = blockIdx.y;
-  int64_t r0 = (int64_t)blockIdx.x * WG_ROWS;
-  int64_t r1 = r0 + WG_ROWS < n_out ? r0 + WG_ROWS : n_out;
+  int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
+  int64_t r1 = r0 + rows_per_block < n_out ? r0 + rows_per_block : n_out;
   int total = Cin * Cout;
   // each thread owns outputs e = threadIdx.x + j*256 (ci = e / Cout, co = e % Cout)
   constexpr int MAXE = 16;  // up to 4096 outputs per pass
@@ -146,19 +147,46 @@ k_wgrad_simt(const float* __restrict__ in, const int32_t* __restrict__ nbr, int6
 #pragma unroll
     for (int j = 0; j < MAXE; ++j) {
       int e = e0 + threadIdx.x + j * 256;
-      if (e < total && acc[j] != 0.f) atomicAdd(dW + (int64_t)k * total + e, acc[j]);
+      if (e < total) part[((int64_t)blockIdx.x * gridDim.y + k) * total + e] = acc[j];
     }
   }
 }
 
+namespace {
+// row chunks of the weight gradient: WG_ROWS rows per block or more, at most about one full wave of blocks in all
+// (8 resident 256-thread blocks per SM) and at most 64 MB of partial dW slots
+int64_t wgrad_simt_chunks(int K, int64_t n_out, int Cin, int Cout) {
+  int64_t chunks = (n_out + WG_ROWS - 1) / WG_ROWS;
+  const int64_t wave = (8 * (int64_t)num_sms() + K - 1) / K;
+  const int64_t mem = (64ll << 20) / ((int64_t)K * Cin * Cout * (int64_t)sizeof(float));
+  if (chunks > wave) chunks = wave;
+  if (chunks > mem) chunks = mem;
+  if (chunks < 1) chunks = 1;
+  const int64_t rows_per_block = (n_out + chunks - 1) / chunks;
+  return (n_out + rows_per_block - 1) / rows_per_block;
+}
+}  // namespace
+
+extern "C" int64_t pasco_conv_wgrad_simt_workspace_bytes(int32_t K, int64_t n_out, int32_t Cin, int32_t Cout) {
+  if (n_out <= 0 || K <= 0 || Cin <= 0 || Cout <= 0) return 0;
+  return wgrad_simt_chunks(K, n_out, Cin, Cout) * K * Cin * Cout * (int64_t)sizeof(float);
+}
+
 extern "C" int pasco_conv_wgrad_simt(const float* in, const int32_t* nbr, int32_t K, int64_t n_out, int32_t Cin,
-                                     int32_t Cout, const float* gout, float* dW, pasco_stream_t s) {
+                                     int32_t Cout, const float* gout, float* dW, float* workspace, int64_t workspace_bytes,
+                                     pasco_stream_t s) {
   if (n_out == 0) return 0;
   size_t smem = (size_t)WG_TILE * (Cin + Cout) * sizeof(float);
   PASCO_CHECK_ARG(smem <= 200 * 1024, "pasco_conv_wgrad_simt: channels too large");
   if (smem > 48 * 1024) cudaFuncSetAttribute(k_wgrad_simt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  dim3 grid((unsigned)((n_out + WG_ROWS - 1) / WG_ROWS), K);
-  k_wgrad_simt<<<grid, 256, smem, (cudaStream_t)s>>>(in, nbr, n_out, Cin, Cout, gout, dW);
+  const int64_t chunks = wgrad_simt_chunks(K, n_out, Cin, Cout);
+  const int64_t rows_per_block = (n_out + chunks - 1) / chunks;
+  const int64_t n_w = (int64_t)K * Cin * Cout;
+  PASCO_CHECK_ARG(workspace && workspace_bytes >= chunks * n_w * (int64_t)sizeof(float),
+                  "pasco_conv_wgrad_simt: workspace smaller than pasco_conv_wgrad_simt_workspace_bytes");
+  dim3 grid((unsigned)chunks, K);
+  k_wgrad_simt<<<grid, 256, smem, (cudaStream_t)s>>>(in, nbr, n_out, Cin, Cout, gout, rows_per_block, workspace);
+  k_add_partials<<<grid_for(n_w, 256), 256, 0, (cudaStream_t)s>>>(workspace, (int)chunks, n_w, n_w, dW);
   PASCO_CHECK_LAUNCH("pasco_conv_wgrad_simt");
   return 0;
 }

@@ -7,7 +7,8 @@
 // A (LBO = distance between two 64-channel sub-tiles) and the gout tile as B (LBO = distance between 64-col blocks).
 // "sub-tile" s = (offset k, 64-channel block cb); a unit = two consecutive sub-tiles = one M=128 accumulator of
 // Cout TMEM columns; a CTA keeps 512/Cout units resident in TMEM, walks its share of 64-row tiles, and finally
-// adds its partial dW with fp32 reductions (red.global.add).
+// stores its partial dW in its own workspace slot; the slots are then added in a fixed order (k_add_partials), so dW
+// is the same from run to run (float atomics would round differently each time).
 #include <stdlib.h>
 #include "common.cuh"
 #include "umma.cuh"
@@ -38,6 +39,7 @@ struct WgradParams {
   int K, Cin, Cout, in_act;
   int stages, tmem_cols;
   int units_per_pass, num_units, num_subs, passes, ctas_per_pass;
+  float* part;  // [ctas_per_pass][K][Cin][Cout] partial dW of each CTA of a pass
 };
 
 constexpr int IDX_RING = 16;   // unit slots are short: fetch neighbour indices 15 slots ahead (HBM-latency bound otherwise)
@@ -288,7 +290,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) k_wgrad_tc(const __grid_consta
     }
 #undef WG_ADV
     cp_async_wait<0>();
-    // epilogue (gather warps 0-3, after their last slot): once the CTA's last MMA has retired, add the partial dW
+    // epilogue (gather warps 0-3, after their last slot): once the CTA's last MMA has retired, store the partial dW
     if (warp < 4) {
     const int q = warp;
     const bool any_work = cta_in_pass < num_rt;
@@ -301,7 +303,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) k_wgrad_tc(const __grid_consta
         const bool ok = sub < p.num_subs;
         const int k = ok ? sub / CB : 0;
         const int cb = ok ? sub - k * CB : 0;
-        float* drow = p.dW + ((int64_t)k * p.Cin + cb * 64 + (L & 63)) * p.Cout;
+        float* drow = p.part + ((int64_t)cta_in_pass * p.K * p.Cin + (int64_t)k * p.Cin + cb * 64 + (L & 63)) * p.Cout;
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(u * p.Cout);
         for (int c0 = 0; c0 < p.Cout; c0 += 32) {
           float v[32];
@@ -309,7 +311,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) k_wgrad_tc(const __grid_consta
           tmem_ld_wait();
           if (ok) {
 #pragma unroll
-            for (int j = 0; j < 32; ++j) atomicAdd(drow + c0 + j, v[j]);
+            for (int j = 0; j < 32; ++j) drow[c0 + j] = v[j];
           }
         }
       }
@@ -387,6 +389,7 @@ struct WgradPlParams {
   int K, Cin, Cout;
   int stages, tmem_cols, depth;
   int units_per_pass, num_units, num_subs, passes, ctas_per_pass;
+  float* part;  // [ctas_per_pass][K][Cin][Cout] partial dW of each CTA of a pass
 };
 
 __device__ __forceinline__ void cp_async16_zfill(uint32_t dst_smem, const void* src, uint32_t src_bytes) {
@@ -554,7 +557,7 @@ __global__ void __launch_bounds__(NUM_THREADS_WPL, 1) k_wgrad_pl(const __grid_co
     }
     cp_async_commit();
     cp_async_wait<0>();
-    // epilogue (gather warps 0-3): once the CTA's last MMA has retired, add the partial dW
+    // epilogue (gather warps 0-3): once the CTA's last MMA has retired, store the partial dW
     if (warp < 4) {
       const int qd = warp;
       if (cta_in_pass < num_rt) {
@@ -566,7 +569,7 @@ __global__ void __launch_bounds__(NUM_THREADS_WPL, 1) k_wgrad_pl(const __grid_co
           const bool ok = sbi < p.num_subs;
           const int k = ok ? sbi / CB : 0;
           const int cb = ok ? sbi - k * CB : 0;
-          float* drow = p.dW + ((int64_t)k * p.Cin + cb * 64 + (L & 63)) * p.Cout;
+          float* drow = p.part + ((int64_t)cta_in_pass * p.K * p.Cin + (int64_t)k * p.Cin + cb * 64 + (L & 63)) * p.Cout;
           const uint32_t taddr = tmem_base + ((uint32_t)(qd * 32) << 16) + (uint32_t)(u * p.Cout);
           for (int c0 = 0; c0 < p.Cout; c0 += 32) {
             float v[32];
@@ -574,7 +577,7 @@ __global__ void __launch_bounds__(NUM_THREADS_WPL, 1) k_wgrad_pl(const __grid_co
             tmem_ld_wait();
             if (ok) {
 #pragma unroll
-              for (int j = 0; j < 32; ++j) atomicAdd(drow + c0 + j, v[j]);
+              for (int j = 0; j < 32; ++j) drow[c0 + j] = v[j];
             }
           }
         }
@@ -647,12 +650,30 @@ int pow2_cols(int c) {
   return v;
 }
 
+// CTAs that share one pass (one set of accumulator units) of either weight-gradient kernel: one partial dW slot each
+int wgrad_ctas_per_pass(int K, int64_t n_out, int Cin, int Cout) {
+  const int num_units = (K * (Cin / 64) + 1) / 2;
+  const int upp = 512 / Cout < num_units ? 512 / Cout : num_units;
+  const int passes = (num_units + upp - 1) / upp;
+  const int64_t num_rt = (n_out + WG_R - 1) / WG_R;
+  int cpp = num_sms() / passes;
+  if (cpp < 1) cpp = 1;
+  if (cpp > num_rt) cpp = (int)num_rt;
+  return cpp;
+}
+
 }  // namespace
+
+extern "C" int64_t pasco_conv_wgrad_workspace_bytes(int32_t K, int64_t n_out, int32_t Cin, int32_t Cout) {
+  if (n_out <= 0 || K <= 0 || Cin < 64 || Cout < 64) return 0;
+  return (int64_t)wgrad_ctas_per_pass(K, n_out, Cin, Cout) * K * Cin * Cout * sizeof(float);
+}
 
 extern "C" int pasco_conv_wgrad_tc(const float* in, int64_t n_in, const int32_t* nbr, int32_t K, int64_t n_out,
                                    int32_t Cin, int32_t Cout, const float* gout, const float* in_scale,
                                    const float* in_shift, int32_t in_act, float* dW, int32_t precision,
-                                   int64_t in_pitch, int64_t gout_pitch, pasco_stream_t s) {
+                                   int64_t in_pitch, int64_t gout_pitch, float* workspace, int64_t workspace_bytes,
+                                   pasco_stream_t s) {
   PASCO_CHECK_ARG(precision == 1 || precision == 3, "pasco_conv_wgrad_tc: precision must be 1 or 3");
   PASCO_CHECK_ARG(Cin % 64 == 0 && Cout % 64 == 0 && Cout <= 256,
                   "pasco_conv_wgrad_tc: Cin (%d) and Cout (%d) must be multiples of 64, Cout <= 256", Cin, Cout);
@@ -686,6 +707,13 @@ extern "C" int pasco_conv_wgrad_tc(const float* in, int64_t n_in, const int32_t*
   if (cpp < 1) cpp = 1;
   if (cpp > num_rt) cpp = (int)num_rt;
   p.ctas_per_pass = cpp;
+  // each CTA stores its partial dW in its own slot (cpp <= num_rt: every CTA has a row tile, so every slot is written in
+  // full); the slots are then summed in a fixed order, which keeps dW identical from run to run
+  const int64_t n_w = (int64_t)K * Cin * Cout;
+  PASCO_CHECK_ARG(cpp == wgrad_ctas_per_pass(K, n_out, Cin, Cout) && workspace &&
+                  workspace_bytes >= (int64_t)cpp * n_w * (int64_t)sizeof(float),
+                  "pasco_conv_wgrad_tc: workspace smaller than pasco_conv_wgrad_workspace_bytes");
+  p.part = workspace;
   const size_t smem = (size_t)2 * g_bytes + (size_t)stages * a_bytes + fixed;
   const int grid = p.passes * cpp;
   cudaError_t e;
@@ -700,13 +728,15 @@ extern "C" int pasco_conv_wgrad_tc(const float* in, int64_t n_in, const int32_t*
     set_error("pasco_conv_wgrad_tc: cudaFuncSetAttribute(%zu bytes) failed: %s", smem, cudaGetErrorString(e));
     return -1;
   }
+  k_add_partials<<<grid_for(n_w, 256), 256, 0, (cudaStream_t)s>>>(p.part, cpp, n_w, n_w, dW);
   PASCO_CHECK_LAUNCH("pasco_conv_wgrad_tc");
   return 0;
 }
 
 extern "C" int pasco_conv_wgrad_planes(const void* in_hi, const void* in_lo, int64_t n_in, const int32_t* nbr, int32_t K,
                                        int64_t n_out, int32_t Cin, int32_t Cout, const void* g_hi, const void* g_lo,
-                                       float* dW, int32_t precision, int64_t in_pitch, int64_t gout_pitch, pasco_stream_t s) {
+                                       float* dW, int32_t precision, int64_t in_pitch, int64_t gout_pitch, float* workspace,
+                                       int64_t workspace_bytes, pasco_stream_t s) {
   PASCO_CHECK_ARG(precision == 1 || precision == 3, "pasco_conv_wgrad_planes: precision must be 1 or 3");
   PASCO_CHECK_ARG(in_hi && g_hi && (precision == 1 || (in_lo && g_lo)), "pasco_conv_wgrad_planes: missing plane");
   PASCO_CHECK_ARG(Cin % 64 == 0 && Cout % 64 == 0 && Cout <= 256,
@@ -773,6 +803,13 @@ extern "C" int pasco_conv_wgrad_planes(const void* in_hi, const void* in_lo, int
   if (cpp < 1) cpp = 1;
   if (cpp > num_rt) cpp = (int)num_rt;
   p.ctas_per_pass = cpp;
+  // each CTA stores its partial dW in its own slot (cpp <= num_rt: every CTA has a row tile, so every slot is written in
+  // full); the slots are then summed in a fixed order, which keeps dW identical from run to run
+  const int64_t n_w = (int64_t)K * Cin * Cout;
+  PASCO_CHECK_ARG(cpp == wgrad_ctas_per_pass(K, n_out, Cin, Cout) && workspace &&
+                  workspace_bytes >= (int64_t)cpp * n_w * (int64_t)sizeof(float),
+                  "pasco_conv_wgrad_planes: workspace smaller than pasco_conv_wgrad_workspace_bytes");
+  p.part = workspace;
   const size_t smem = (size_t)2 * g_bytes + (size_t)stages * a_bytes + fixed;
   const int grid = p.passes * cpp;
   cudaError_t e;
@@ -787,6 +824,7 @@ extern "C" int pasco_conv_wgrad_planes(const void* in_hi, const void* in_lo, int
     set_error("pasco_conv_wgrad_planes: cudaFuncSetAttribute(%zu bytes) failed: %s", smem, cudaGetErrorString(e));
     return -1;
   }
+  k_add_partials<<<grid_for(n_w, 256), 256, 0, (cudaStream_t)s>>>(p.part, cpp, n_w, n_w, dW);
   PASCO_CHECK_LAUNCH("pasco_conv_wgrad_planes");
   return 0;
 }

@@ -11,7 +11,8 @@
 //   PASS 0  S = Q_h·K_hᵀ per 64-key tile (tcgen05, M=128 queries, N=64 keys, K=64 padded head dim) → per (chunk, h, q)
 //           running max m and Σ exp(s − m); `k_xattn_lse` merges the chunks into lse[h, q].
 //   PASS 1  S again, p = exp(s − lse) (already normalised), P → bf16 (hi+lo) K-major smem tile, O_h += P·V_h (tcgen05,
-//           V tile as MN-major B operand), accumulated in TMEM over all tiles of the CTA, then fp32 red.add into O.
+//           V tile as MN-major B operand), accumulated in TMEM over all tiles of the CTA, then stored as the chunk's
+//           partial O in the workspace; the chunks are added into O in chunk order (k_add_partials).
 // A CTA = (head, key chunk); warps 0-3: one query row per thread (TMEM lane = row; mask, exp, row statistics),
 // warps 4-7: K/V tile gather (16 lanes per 256-byte padded row segment, fp32 → bf16 hi/lo split, 128-byte swizzle),
 // warp 8: single-thread MMA issue.  Operands are split bf16x3 like the convolution ("fp32" mode).
@@ -39,7 +40,7 @@ struct XParams {
   const uint32_t* mask; // bit rows [Q, 2*ceil(P/64)]: bit j of word 2t + j/32 = key 64t + j masked; nullptr = none
   const float* lse;    // [H, Q]            (pass 1)
   float* out;          // [Q, H*D] zeroed   (pass 1)
-  float* ws;           // [chunks, H, Q, 2] (pass 0)
+  float* ws;           // [chunks, H, Q, 2] (pass 0), then [chunks, Q, H*D] per-chunk outputs (pass 1)
   int Q, H, D;
   int64_t P;
   int chunks;
@@ -306,13 +307,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_xattn_fwd(const __grid_constant
       tmem_ld32(taddr + 32, b);
       tmem_ld_wait();
       if (qok) {
-        float* orow = p.out + (int64_t)qrow * HD + h * p.D;
+        float* orow = p.ws + (int64_t)p.chunks * p.H * p.Q * 2 + ((int64_t)chunk * p.Q + qrow) * HD + h * p.D;
 #pragma unroll
         for (int d = 0; d < 32; ++d)
-          if (d < p.D) atomicAdd(orow + d, a[d]);
+          if (d < p.D) orow[d] = a[d];
 #pragma unroll
         for (int d = 0; d < 32; ++d)
-          if (32 + d < p.D) atomicAdd(orow + 32 + d, b[d]);
+          if (32 + d < p.D) orow[32 + d] = b[d];
       }
     }
   }
@@ -344,11 +345,17 @@ int pick_chunks(int64_t P, int H) {
   return c < 1 ? 1 : c;
 }
 
+// key chunks that own at least one tile (the kernels' split: ceil(tiles / chunks) tiles per chunk); only these write
+// their slot of per-chunk partial sums
+int live_chunks(int64_t P, int chunks) {
+  const int64_t tiles = (P + BK - 1) / BK, per = (tiles + chunks - 1) / chunks;
+  return (int)((tiles + per - 1) / per);
+}
+
 }  // namespace
 
 extern "C" int64_t pasco_xattn_workspace_bytes(int32_t Q, int64_t P, int32_t H, int32_t D) {
-  (void)D;
-  return (int64_t)pick_chunks(P, H) * H * Q * 2 * sizeof(float);
+  return (int64_t)pick_chunks(P, H) * (H * Q * 2 + (int64_t)Q * H * D) * sizeof(float);
 }
 
 extern "C" int pasco_xattn_forward(const float* q, const float* k, const float* v, const uint32_t* mask, int32_t Q,
@@ -374,6 +381,10 @@ extern "C" int pasco_xattn_forward(const float* q, const float* k, const float* 
   k_xattn_fwd<0><<<grid, NTHREADS, SMEM_BYTES, st>>>(p);
   k_xattn_lse<<<(H * Q + 127) / 128, 128, 0, st>>>(workspace, p.chunks, H * Q, lse);
   k_xattn_fwd<1><<<grid, NTHREADS, SMEM_BYTES, st>>>(p);
+  // the chunks' partial outputs summed in chunk order (identical from run to run, unlike float atomics)
+  const int64_t n_o = (int64_t)Q * H * D;
+  k_add_partials<<<grid_for(n_o, 256), 256, 0, st>>>(workspace + (int64_t)p.chunks * H * Q * 2, live_chunks(P, p.chunks),
+                                                     n_o, n_o, out);
   PASCO_CHECK_LAUNCH("pasco_xattn_forward");
   return 0;
 }
@@ -390,7 +401,7 @@ extern "C" int pasco_xattn_forward(const float* q, const float* k, const float* 
 //   dKᵀ[ 64d x 64k] = Qsᵀ(MN-major, zero-padded)            · dS(MN-major)
 //   dQ [128q x 64d] += dS(K-major) · K(MN-major)              (accumulates in TMEM over the CTA's tiles)
 // dVᵀ/dKᵀ land with lane = head-dim index, so one warp store writes 32 consecutive floats of a key's row:
-// every dK/dV row is written exactly once (no atomics); dQ is added with fp32 red.add at the end.
+// every dK/dV row is written exactly once (no atomics); each chunk stores its dQ, and the chunks are summed in order.
 // ==================================================================================================================
 namespace {
 
@@ -398,6 +409,7 @@ struct XBwdParams {
   const float* q; const float* k; const float* v; const uint32_t* mask; const float* lse;
   const float* out; const float* dout;
   float* dq; float* dk; float* dv;
+  float* dq_part;      // [chunks, Q, H*D] dQ of each key chunk
   int Q, H, D;
   int64_t P;
   int chunks;
@@ -705,13 +717,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_xattn_bwd(const __grid_constant
       tmem_ld32(taddr + 32, b);
       tmem_ld_wait();
       if (qok) {
-        float* row = p.dq + (int64_t)qrow * HD + h * p.D;
+        float* row = p.dq_part + ((int64_t)chunk * p.Q + qrow) * HD + h * p.D;
 #pragma unroll
         for (int d = 0; d < 32; ++d)
-          if (d < p.D) atomicAdd(row + d, a[d] * p.scale);
+          if (d < p.D) row[d] = a[d] * p.scale;
 #pragma unroll
         for (int d = 0; d < 32; ++d)
-          if (32 + d < p.D) atomicAdd(row + 32 + d, b[d] * p.scale);
+          if (32 + d < p.D) row[32 + d] = b[d] * p.scale;
       }
     }
   }
@@ -727,7 +739,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_xattn_bwd(const __grid_constant
 
 extern "C" int pasco_xattn_backward(const float* q, const float* k, const float* v, const uint32_t* mask, const float* lse,
                                     const float* out, const float* dout, int32_t Q, int64_t P, int32_t H, int32_t D,
-                                    float scale, float* dq, float* dk, float* dv, pasco_stream_t s) {
+                                    float scale, float* dq, float* dk, float* dv, float* workspace,
+                                    int64_t workspace_bytes, pasco_stream_t s) {
   PASCO_CHECK_ARG(Q >= 1 && Q <= QM, "pasco_xattn_backward: Q (%d) must be in [1,128]", Q);
   PASCO_CHECK_ARG(D >= 4 && D <= DP && D % 4 == 0, "pasco_xattn_backward: head dim (%d) must be a multiple of 4, <= 64", D);
   PASCO_CHECK_ARG((((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)dq | (uintptr_t)dk | (uintptr_t)dv) & 15) == 0,
@@ -737,12 +750,18 @@ extern "C" int pasco_xattn_backward(const float* q, const float* k, const float*
   p.dq = dq; p.dk = dk; p.dv = dv;
   p.Q = Q; p.H = H; p.D = D; p.P = P; p.scale = scale;
   p.chunks = pick_chunks(P, H);
+  const int64_t n_q = (int64_t)Q * H * D;
+  const int n_live = live_chunks(P, p.chunks);
+  PASCO_CHECK_ARG(workspace && workspace_bytes >= (int64_t)n_live * n_q * (int64_t)sizeof(float),
+                  "pasco_xattn_backward: workspace smaller than pasco_xattn_workspace_bytes");
+  p.dq_part = workspace;
   cudaError_t e = cudaFuncSetAttribute(k_xattn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, B_SMEM_BYTES);
   if (e != cudaSuccess) {
     set_error("pasco_xattn_backward: cudaFuncSetAttribute(%d) failed: %s", B_SMEM_BYTES, cudaGetErrorString(e));
     return -1;
   }
   k_xattn_bwd<<<p.chunks * H, NTHREADS, B_SMEM_BYTES, (cudaStream_t)s>>>(p);
+  k_add_partials<<<grid_for(n_q, 256), 256, 0, (cudaStream_t)s>>>(p.dq_part, n_live, n_q, n_q, dq);
   PASCO_CHECK_LAUNCH("pasco_xattn_backward");
   return 0;
 }

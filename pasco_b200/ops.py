@@ -470,6 +470,11 @@ def fuse_bn_stats(flag: bool) -> None:
     _FUSE_BN_STATS = bool(flag)
 
 
+def _workspace(nbytes: int, device) -> torch.Tensor:
+    """Scratch memory for a library call, from the caching allocator (stream-ordered like the call itself)."""
+    return torch.empty(max(nbytes // 4, 1), dtype=torch.float32, device=device)
+
+
 def conv_wgrad(feats: torch.Tensor, gout: torch.Tensor, nbr: Optional[torch.Tensor], K: int, Cin: int, Cout: int,
                in_scale=None, in_shift=None, in_act: int = 0, in_planes=None, g_planes=None) -> torch.Tensor:
     """in_planes / g_planes: (hi, lo) bf16 planes of act(feats·scale+shift) and of gout when the caller has them
@@ -483,19 +488,25 @@ def conv_wgrad(feats: torch.Tensor, gout: torch.Tensor, nbr: Optional[torch.Tens
         ev0.record()
     tc = _tc_ok(Cin, 64, 1, "wgrad") and Cin % 64 == 0 and Cout % 64 == 0 and Cout <= 256
     path = "planes" if tc and _planes_ok(Cin, K, nbr) else ("regs" if tc else "simt")
+    if tc:
+        # per-CTA partial dW, summed in a fixed order by the library (dW does not change from run to run)
+        nbytes = _lib.load().pasco_conv_wgrad_workspace_bytes(K, n_out, Cin, Cout)
+        ws = _workspace(nbytes, feats.device)
     if tc and _planes_ok(Cin, K, nbr):
         ih, il = in_planes if in_planes is not None else split_planes(feats, in_scale, in_shift, in_act)
         gh, gl = g_planes if g_planes is not None else split_planes(gout)
         call("pasco_conv_wgrad_planes", ptr(ih), ptr(il), feats.shape[0], ptr(nbr), K, n_out, Cin, Cout, ptr(gh), ptr(gl),
-             ptr(dW), _PRECISION, 0, 0)
+             ptr(dW), _PRECISION, 0, 0, ptr(ws), nbytes)
     elif tc:
         call("pasco_conv_wgrad_tc", ptr(feats), feats.shape[0], ptr(nbr), K, n_out, Cin, Cout, ptr(gout),
-             ptr(in_scale), ptr(in_shift), in_act, ptr(dW), _PRECISION, 0, 0)
+             ptr(in_scale), ptr(in_shift), in_act, ptr(dW), _PRECISION, 0, 0, ptr(ws), nbytes)
     else:
         assert in_scale is None and in_act == 0
         if nbr is None:
             nbr = torch.arange(n_out, dtype=torch.int32, device=feats.device).view(1, -1)
-        call("pasco_conv_wgrad_simt", ptr(feats), ptr(nbr), K, n_out, Cin, Cout, ptr(gout), ptr(dW))
+        nbytes = _lib.load().pasco_conv_wgrad_simt_workspace_bytes(K, n_out, Cin, Cout)
+        ws = _workspace(nbytes, feats.device)
+        call("pasco_conv_wgrad_simt", ptr(feats), ptr(nbr), K, n_out, Cin, Cout, ptr(gout), ptr(dW), ptr(ws), nbytes)
     if prof is not None:
         ev1 = torch.cuda.Event(enable_timing=True)
         ev1.record()
@@ -816,8 +827,10 @@ class MaskedCrossAttention(torch.autograd.Function):
         go = go.contiguous().float()
         dq = torch.zeros_like(q)
         dk, dv = torch.empty_like(k), torch.empty_like(v)
+        nbytes = _lib.load().pasco_xattn_workspace_bytes(Q, P, H, HD // H)
+        ws = _workspace(nbytes, q.device)
         call("pasco_xattn_backward", ptr(q), ptr(k), ptr(v), ptr(bits), ptr(lse), ptr(out), ptr(go), Q, P, H, HD // H,
-             C.c_float(scale), ptr(dq), ptr(dk), ptr(dv))
+             C.c_float(scale), ptr(dq), ptr(dk), ptr(dv), ptr(ws), nbytes)
         return dq, dk, dv, None, None
 
 
@@ -875,8 +888,10 @@ class LinearTC(torch.autograd.Function):
             for c0 in range(0, cin, 256):                                        # dW[:, c0:c0+cw] = gyᵀ @ x[:, c0:c0+cw]
                 cw = min(256, cin - c0)
                 dw = torch.zeros(1, cout, cw, dtype=torch.float32, device=x.device)
+                nbytes = _lib.load().pasco_conv_wgrad_workspace_bytes(1, gy.shape[0], cout, cw)
+                ws = _workspace(nbytes, x.device)
                 call("pasco_conv_wgrad_tc", ptr(gy), gy.shape[0], None, 1, gy.shape[0], cout, cw,
-                     C.c_void_p(_data_ptr_at(x, c0)), None, None, 0, ptr(dw), _PRECISION, 0, cin)
+                     C.c_void_p(_data_ptr_at(x, c0)), None, None, 0, ptr(dw), _PRECISION, 0, cin, ptr(ws), nbytes)
                 gw[:, c0:c0 + cw] = dw[0]
         if ctx.has_bias and ctx.needs_input_grad[2]:
             gb = gy.sum(0)

@@ -1,12 +1,12 @@
-"""The real drop-in: the UNMODIFIED reference model (`pasco.models.net_panoptic_sparse.Net`, staged by
-tools/stage_reference.py under baseline/_ref/, which ships to the GPU box but is never committed) runs on the B200
-with `import MinkowskiEngine` / `torch_scatter` resolving to compat/ → pasco_b200.me → libpasco_sm100.so, and its
-outputs are compared (a) with the golden vectors the same reference produced on the CPU oracle and (b) with the
-engine-native PascoNet on the same weights and scene.
+"""The real drop-in: the UNMODIFIED reference model (`pasco.models.net_panoptic_sparse.Net`, compiled by build() from an
+upstream PaSCo checkout into oracle/_ref/, which is not committed) runs on the B200 with `import MinkowskiEngine` /
+`torch_scatter` resolving to compat/ → pasco_b200.me → libpasco_sm100.so, and its outputs are compared (a) with the
+golden vectors the same reference produced on the CPU oracle and (b) with the engine-native PascoNet on the same
+weights and scene.
 
 Reference path exercised: net_panoptic_sparse.py:210-312 → unet3d_sparse_v2.py:216-256 (encoder_v2, dense bottleneck
 through nn.Conv3d, decoder_v3 incl. predict_completion_sem_logit / predict_panop, transformer_predictor_v2).
-Skips cleanly when baseline/_ref is absent.
+PASCO_REFERENCE (the root of an upstream checkout) overrides oracle/_ref; the tests skip when neither holds `pasco/`.
 """
 import json
 import os
@@ -18,13 +18,14 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.environ.get("PASCO_REFERENCE") or os.path.join(ROOT, "oracle", "_ref")
 sys.path.insert(0, os.path.join(HERE, "golden"))
 from recipe import fill_state_dict  # noqa: E402
 from test_golden_net import _compare  # noqa: E402
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pasco")), reason="baseline/_ref not staged")]
+              pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pasco")),
+                                 reason="no upstream PaSCo package: build() compiles one into oracle/_ref from a checkout")]
 
 
 def _reference_net(n_infers=1, heavy=False, n_classes=20, in_channels=283):
