@@ -240,6 +240,37 @@ int pasco_xattn_backward(const float* q, const float* k, const float* v, const u
                          const float* out, const float* dout, int32_t Q, int64_t P, int32_t H, int32_t D, float scale,
                          float* dq, float* dk, float* dv, float* workspace, int64_t workspace_bytes, pasco_stream_t s);
 
+/* ---- evaluation (pasco/models/metrics.py SSCMetrics + UncertaintyMetrics, pasco/loss/panoptic_quality.py) ---------
+ * Calibration binning is torchmetrics' binary_calibration_error: bounds = torch.linspace(0, 1, n_bins + 1) in fp32,
+ * slot = bucketize(conf, bounds, right=True) - 1 over n_bins + 1 slots (NB below).  Integer outputs are ACCUMULATED
+ * (+=, the caller zeroes them once); fp64 sums are accumulated too and are the same from run to run.  A label >= K
+ * (other than 255 = unknown) or a segment id outside its table sets *err_flag = 3 and the cell or row is skipped.
+ *
+ * One sweep over a scene's cells: prob float [K, cells] (class-major, empty cells one-hot class 0), label uint8 [cells].
+ * Per cell: pred = argmax (first maximum), conf = max prob.
+ * Everything is over known cells (SSCMetrics.add_batch zeroes unknown cells, then masks them out).
+ *   counts int64 [K*K + 4*NB]: confusion[target][pred] (SSCMetrics.add_batch), then split by pred == 0 / pred != 0:
+ *     calibration counts [2][NB], correct (pred == label) counts [2][NB];
+ *   sums double [2*NB + 2]: Σ conf [2][NB], Σ -log(p[label] + 1e-12) [2] (add_batch_ece).                           */
+int64_t pasco_eval_ssc_workspace_bytes(int64_t cells, int32_t n_bins);
+int pasco_eval_ssc(const float* prob, const uint8_t* label, int64_t cells, int32_t K, const float* bounds,
+                   int32_t n_bins, int64_t* counts, double* sums, double* workspace, int64_t workspace_bytes,
+                   int32_t* err_flag, pasco_stream_t s);
+/* Intersection table of GT panoptic ids (gt_id int32 [cells], 0..n_gt) and predicted ids (pred_id int32 [n_rows],
+ * 0..n_pred, at cell row_cell[r]; cells without a row are id 0) over known cells: table int64 [(n_gt+1) * (n_pred+1)].
+ * Column sums are the predicted areas, row sums the GT areas, both after unknown cells are zeroed.                  */
+int pasco_eval_pairs(const int32_t* pred_id, const int64_t* row_cell, int64_t n_rows, const int32_t* gt_id,
+                     const uint8_t* label, int64_t cells, int32_t n_gt, int32_t n_pred, int64_t* table, int32_t* err_flag,
+                     pasco_stream_t s);
+/* Binned calibration of per-row mask confidences (UncertaintyMetrics.compute_ece_panop): rows whose cell is known with
+ * gt_id != 0 and conf != 0; correct when match[pred_id] (int32 [n_pred+1], the GT id matched to each predicted
+ * segment, 0 = none) == gt_id.  counts int64 [2*NB] (count, correct), sums double [NB] (Σ conf).                     */
+int64_t pasco_eval_calib_workspace_bytes(int64_t n_rows, int32_t n_bins);
+int pasco_eval_calib(const float* conf, const int32_t* pred_id, const int64_t* row_cell, int64_t n_rows,
+                     const int32_t* gt_id, const uint8_t* label, int64_t cells, const int32_t* match, int32_t n_pred,
+                     const float* bounds, int32_t n_bins, int64_t* counts, double* sums, double* workspace,
+                     int64_t workspace_bytes, int32_t* err_flag, pasco_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif

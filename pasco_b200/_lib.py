@@ -62,6 +62,11 @@ PROTOTYPES = {
     "pasco_xattn_forward": (C.c_int, [_p, _p, _p, _p, _i32, _i64, _i32, _i32, C.c_float, _p, _p, _p, _i64, _p]),
     "pasco_xattn_backward": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _i64, _i32, _i32, C.c_float, _p, _p, _p, _p, _i64, _p]),
     "pasco_bn_bwd_apply": (C.c_int, [_p, _p, _i64, _i32, _p, _p, _i32, _p, _p, _p, _p, _p]),
+    "pasco_eval_ssc_workspace_bytes": (_i64, [_i64, _i32]),
+    "pasco_eval_ssc": (C.c_int, [_p, _p, _i64, _i32, _p, _i32, _p, _p, _p, _i64, _p, _p]),
+    "pasco_eval_pairs": (C.c_int, [_p, _p, _i64, _p, _p, _i64, _i32, _i32, _p, _p, _p]),
+    "pasco_eval_calib_workspace_bytes": (_i64, [_i64, _i32]),
+    "pasco_eval_calib": (C.c_int, [_p, _p, _p, _i64, _p, _p, _i64, _p, _i32, _p, _i32, _p, _p, _p, _i64, _p, _p]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -904,3 +904,41 @@ def linear(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor] =
     if x.is_cuda and x.ndim == 2 and _linear_tc_ok(x.shape[0], weight.shape[1], weight.shape[0]):
         return LinearTC.apply(x, weight, bias)
     return torch.nn.functional.linear(x, weight, bias)
+
+
+# ----------------------------------------------------------------------------------------------
+# evaluation sweeps (pasco_b200/evaluation.py): outputs are accumulated into caller-zeroed tensors
+# ----------------------------------------------------------------------------------------------
+EVAL_ERR_ID = 3         # _err_flag code of the evaluation kernels: a label or segment id outside its table
+
+
+def eval_ssc(prob: torch.Tensor, label: torch.Tensor, bounds: torch.Tensor, counts: torch.Tensor,
+             sums: torch.Tensor) -> None:
+    """prob float32 [K, cells], label uint8 [cells]; counts int64 [K*K + 4*(n_bins+1)], sums float64
+    [2*(n_bins+1) + 2] (layouts: include/pasco_sm100.h)."""
+    K, cells = prob.shape
+    n_bins = bounds.numel() - 1
+    nbytes = _lib.load().pasco_eval_ssc_workspace_bytes(cells, n_bins)
+    ws = _workspace(nbytes, prob.device)
+    call("pasco_eval_ssc", ptr(prob), ptr(label), cells, K, ptr(bounds), n_bins, ptr(counts), ptr(sums), ptr(ws), nbytes,
+         ptr(_err_flag(prob.device)))
+
+
+def eval_pairs(pred_id: torch.Tensor, row_cell: torch.Tensor, gt_id: torch.Tensor, label: torch.Tensor, n_gt: int,
+               n_pred: int, table: torch.Tensor) -> None:
+    """table int64 [(n_gt+1) * (n_pred+1)] += intersections of GT ids (gt_id int32 [cells]) and predicted ids
+    (pred_id int32 [N] at cells row_cell int64 [N]) over known cells."""
+    call("pasco_eval_pairs", ptr(pred_id), ptr(row_cell), pred_id.numel(), ptr(gt_id), ptr(label), gt_id.numel(),
+         int(n_gt), int(n_pred), ptr(table), ptr(_err_flag(gt_id.device)))
+
+
+def eval_calib(conf: torch.Tensor, pred_id: torch.Tensor, row_cell: torch.Tensor, gt_id: torch.Tensor,
+               label: torch.Tensor, match: torch.Tensor, bounds: torch.Tensor, counts: torch.Tensor,
+               sums: torch.Tensor) -> None:
+    """Binned calibration of the rows' mask confidences; match int32 [n_pred+1] = GT id matched to each predicted id."""
+    n_bins = bounds.numel() - 1
+    nbytes = _lib.load().pasco_eval_calib_workspace_bytes(conf.numel(), n_bins)
+    ws = _workspace(nbytes, conf.device)
+    call("pasco_eval_calib", ptr(conf), ptr(pred_id), ptr(row_cell), conf.numel(), ptr(gt_id), ptr(label), gt_id.numel(),
+         ptr(match), match.numel() - 1, ptr(bounds), n_bins, ptr(counts), ptr(sums), ptr(ws), nbytes,
+         ptr(_err_flag(conf.device)))
